@@ -108,6 +108,27 @@ def make_descs_fast(abi, G, R, gid0=0, name0=0, prefix="NoopPaxosApp", version=0
     return d
 
 
+DUMP_LIMIT = 64_000_000  # bytes of all files together
+
+
+def dump_round_outputs(out_dir, abi, status, exec_bytes, R):
+    """What one gpx_round_device call returned, as float64 arrays under out_dir, one file per field: status [G] and the
+    EXEC records [G, R] (req_id split into 32-bit halves, which float64 holds exactly).  When that exceeds DUMP_LIMIT,
+    the same fields for a fixed sample of the groups (seed 0), whose indices go to group_index.npy."""
+    ex = exec_bytes.view(abi.exec_dtype).reshape(-1, R)
+    cols = {"status": status, "exec_gid": ex["gid"], "exec_slot": ex["slot"], "exec_req_id_hi": ex["req_id"] >> 32,
+            "exec_req_id_lo": ex["req_id"] & 0xFFFFFFFF, "exec_payload_off": ex["payload_off"], "exec_flags": ex["flags"]}
+    G, per_group = len(status), 8 * (1 + 6 * R)
+    idx = np.arange(G)
+    if G * per_group > DUMP_LIMIT:
+        idx = np.sort(np.random.default_rng(0).choice(G, size=(DUMP_LIMIT - 4096) // (per_group + 8), replace=False))
+        cols = {name: a[idx] for name, a in cols.items()}
+        cols["group_index"] = idx
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in cols.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, dtype=np.float64))
+
+
 def hbm_peak():
     p = os.path.join(ROOT, "MEASURED_PEAKS.json")
     if os.path.exists(p):
@@ -380,7 +401,13 @@ def main():
                     help="spread: store the records straight into the peers' receive buckets over NVLink (GPX_SPREAD_P2P, CUDA "
                          "IPC between the ranks) instead of exchanging the buckets with grouped ncclSend/ncclRecv; falls back "
                          "to the NCCL exchange when the peer mapping cannot be set up")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps write what the last one returned (status and EXEC records of rank 0's "
+                         "groups) as DIR/<name>.npy in float64, a fixed sample of the groups beyond 64 MB; "
+                         "packed placement, workloads cfg2, cfg3 and 1m1b")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
 
     wl = dict(WORKLOADS[args.workload])
     if args.groups:
@@ -394,6 +421,8 @@ def main():
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     if args.placement == "auto":
         args.placement = "spread" if (world >= R and world > 1) else "packed"
+    if args.dump_outputs and (args.impl != "ours" or args.placement != "packed" or args.workload in ("cfg4", "cfg5")):
+        ap.error("--dump-outputs covers the packed round path of workloads cfg2, cfg3 and 1m1b")
     metric = "paxos_decisions_per_sec"
     config = {
         "workload": wl["name"], "groups_per_gpu": G, "replicas": R, "payload_bytes": P, "window": 8,
@@ -515,6 +544,8 @@ def main():
     assert decided == G * K, f"expected {G * K} decisions in the timed region, engine made {decided}"
     assert c1["executed"] - c0["executed"] == G * K * R
     value = world * G * K / (total_ms / 1e3)
+    if args.dump_outputs and rank == 0:  # before the legs below reuse d_status / d_exec
+        dump_round_outputs(args.dump_outputs, abi, d_status.cpu().numpy(), d_exec.cpu().numpy(), R)
 
     # ---- roofline: per-kernel CUDA events inside the engine (same launches, same stream) ----
     def kernel_times(fn_name, K2):

@@ -385,8 +385,8 @@ class PaxosManager:
                         if int(c["kind"]) == abi.CO_PVALUE and int(c["pv"]["payload_len"]):
                             per_lane.setdefault(int(c["src_reply"]) % L, []).append((n, j, c["pv"]))
                 for l, items in per_lane.items():
-                    got = eng.log_gather(l, [int(pv["frame_ref"]) * 16 for _, _, pv in items],
-                                         [int(pv["payload_len"]) for _, _, pv in items])
+                    pos = self._blob_positions(l, [(self.instances[n].gid, pv) for n, _, pv in items])
+                    got = eng.log_gather(l, pos, [int(pv["payload_len"]) for _, _, pv in items])
                     for (n, j, _), b in zip(items, got):
                         body_of[(n, j)] = b
             for j in range(max((len(p) for p in plans.values()), default=0)):
@@ -611,10 +611,76 @@ class PaxosManager:
             plan = plan + [(next_slot, abi.CO_STOP_NEW, None, 0)]
         return plan, flags
 
+    def _blob_positions(self, lane: int, items) -> List[int]:
+        """the log positions (for gpx_log_read / gpx_log_gather) of the request blobs of carried-over pvalues, given as
+        [(gid, accepted pvalue)] reported by the acceptor at `lane`.  frame_ref * 16 is the blob's offset in the lane's
+        ring of log_ring_bytes: until the ring has wrapped that is its position.  After that the offset does not say
+        which lap wrote it, so the ACCEPT that logged the pvalue is looked up among the bytes still in the ring
+        (gpx_log_find from the oldest intact segment boundary) and its blob position taken.  A pvalue whose ACCEPT is
+        no longer there raises GPX_ERANGE: its body was overwritten."""
+        eng = self.engine
+        head, ring = eng.log_head(lane), int(eng.cfg.log_ring_bytes)
+        if head <= ring:
+            return [int(pv["frame_ref"]) * 16 for _, pv in items]
+        start = self._oldest_segment(lane, head, ring)
+        todo: Dict[int, List[int]] = {}
+        for gid, pv in items:
+            todo.setdefault(int(gid), []).append(int(pv["slot"]))
+        for g, sl in todo.items():
+            todo[g] = sorted(set(sl), key=lambda s, s0=sl[0]: _jsub(s, s0))
+        hits = {}
+        while todo:  # one want per group and call, GPX_LOG_SPAN slots from its lowest slot still to find
+            gids = sorted(todo)
+            w = np.zeros(len(gids), dtype=abi.log_want_dtype)
+            w["gid"], w["min_slot"], w["n_slots"] = gids, [todo[g][0] for g in gids], abi.GPX_LOG_SPAN
+            found = eng.log_find(lane, w, start)
+            for i, g in enumerate(gids):
+                s0 = todo[g][0]
+                for s in todo[g]:
+                    if _jsub(s, s0) < abi.GPX_LOG_SPAN:
+                        hits[(g, s)] = found[i, _jsub(s, s0)]
+                todo[g] = [s for s in todo[g] if _jsub(s, s0) >= abi.GPX_LOG_SPAN]
+                if not todo[g]:
+                    del todo[g]
+        out = []
+        for gid, pv in items:
+            h = hits[(int(gid), int(pv["slot"]))]
+            a = h["accept"]
+            same = all(int(a[f]) == int(pv[f]) for f in ("bnum", "bcoord", "req_id", "payload_len"))
+            if int(a["flags"]) & abi.F_VOID or not same:
+                raise abi.GpxError(abi.GPX_ERANGE, f"the request body of group {int(gid)} slot {int(pv['slot'])} "
+                                                   f"at lane {lane} was overwritten in the log ring")
+            out.append(int(h["blob_pos"]))
+        return out
+
+    def _oldest_segment(self, lane: int, head: int, ring: int) -> int:
+        """the first segment boundary among the last `ring` bytes before the head of a lane's log: a segment header
+        names its own absolute position (ring_off), and the walk from the boundary over the headers (to the next lap
+        where a launch skipped the ring end, as k_log_dir walks) ends at the head"""
+        buf = self.engine.log_read(lane, head - ring, ring)
+        n = ring // 32 - 1
+        hdr = np.lib.stride_tricks.as_strided(buf, shape=(n, 64), strides=(32, 1)).copy().view(abi.seg_hdr_dtype)[:, 0]
+        pos = head - ring + 32 * np.arange(n, dtype=np.int64)
+        ok = (hdr["magic"] == abi.SEG_MAGIC) & (hdr["ring_off"] == pos.astype(np.uint64)) & (pos % ring + 64 <= ring)
+        for k in np.nonzero(ok)[0]:
+            p = int(pos[k])
+            while p + 64 <= head:
+                i = (p - (head - ring)) // 32
+                if i < n and ok[i]:
+                    h = hdr[i]
+                    body = int(h["n_slots"]) * int(h["rec_bytes"]) + ((int(h["payload_bytes"]) + 15) & ~15)
+                    p = (p + 64 + body + 31) & ~31
+                else:  # the tail a launch skipped at the ring end
+                    p = (p // ring + 1) * ring
+            if p == head:
+                return int(pos[k])
+        raise abi.GpxError(abi.GPX_ERANGE, f"no intact segment boundary in the log ring of lane {lane}")
+
     def _requests_of(self, paxosID: str, pv, src_lane: int, entry: int) -> List[RequestPacket]:
         """the request(s) of an accepted pvalue, read back from the log ring of the acceptor lane that reported it"""
         n = int(pv["payload_len"])
-        blob = bytes(self.engine.log_read(src_lane, int(pv["frame_ref"]) * 16, n)) if n else b""
+        pos = self._blob_positions(src_lane, [(self.instances[paxosID].gid, pv)])[0] if n else 0
+        blob = bytes(self.engine.log_read(src_lane, pos, n)) if n else b""
         return self._requests_from_blob(paxosID, pv, blob, entry)
 
     # ---- catching up a replica that fell behind (PISM.syncLongDecisionGaps :1550, checkpoint transfer :1852) ----

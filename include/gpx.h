@@ -378,7 +378,7 @@ typedef struct gpx_accepted_pvalue { /* one accepted pvalue of a PREPARE_REPLY, 
   int32_t slot;
   int32_t bnum;
   int32_t bcoord;
-  uint32_t frame_ref;   /* log ring position / 16 of the request blob at this acceptor */
+  uint32_t frame_ref;   /* offset / 16 of the request blob in this acceptor's log ring (which wraps) */
   int64_t req_id;
   uint32_t payload_len;
   uint32_t flags;       /* bit1 STOP, bits 16.. nreq */
@@ -417,7 +417,7 @@ int gpx_handle_prepares(gpx_engine* e, uint32_t n, const gpx_pvalue_hdr* prepare
  *       other local lanes resign (PISM.handlePrepare would have removed them when the PREPARE arrived).
  * The plan is returned, not proposed: spawnCommandersForProposals :556-575 is the caller re-proposing plan[0..n_plan)
  * in order through gpx_propose / gpx_round (the request bodies of a carried-over pvalue are in the log ring of the
- * acceptor that reported it: reply index src_reply, position frame_ref * 16).  The engine keeps no pre-active
+ * acceptor that reported it: reply index src_reply, ring offset frame_ref * 16).  The engine keeps no pre-active
  * proposals (a request that finds a pre-active coordinator gets GPX_RS_PREACTIVE and waits at the host), so
  * combinePValuesOntoProposals' preActives and reproposePreemptedProposals :460-468 have nothing to do here.
  *
@@ -595,10 +595,10 @@ typedef struct gpx_log_hit { /* 96 B */
 } gpx_log_hit;
 int gpx_log_find(gpx_engine* e, uint32_t lane, uint64_t from, uint32_t n, const gpx_log_want* wants, gpx_log_hit* out);
 
-/* Request bodies for a batch of gpx_log_find hits (or of carried-over pvalues: position = frame_ref * 16) in ONE
- * device->host copy: ranges[i] = {ring position, length, offset in dst (a multiple of 16)}; range i lands at
- * dst + dst_off rounded up to whole 16-byte chunks (the ring's payload areas are padded to 16).  The journal analogue is
- * SQLPaxosLogger.getJournaledMessage(FileOffsetLength[]) :3712, which reads the indexed frames back in one pass. */
+/* Request bodies for a batch of gpx_log_find hits (or of carried-over pvalues: ring offset frame_ref * 16, which is the
+ * position until the ring wraps) in ONE device->host copy: ranges[i] = {ring position, length, offset in dst (a multiple
+ * of 16)}; range i lands at dst + dst_off rounded up to whole 16-byte chunks (the ring's payload areas are padded to
+ * 16).  The journal analogue is SQLPaxosLogger.getJournaledMessage(FileOffsetLength[]) :3712 (frames in one pass). */
 typedef struct gpx_log_range { /* 16 B */
   uint64_t pos;
   uint32_t len;

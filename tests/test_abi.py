@@ -97,12 +97,11 @@ def test_properties_parser(cuda_lib, tmp_path):
     assert cuda_lib.fn("properties_actives")(buf, C.c_size_t(1024)) == 0
     assert buf.value.decode().splitlines() == ["100=127.0.0.1:2000", "101=127.0.0.1:2001", "102=127.0.0.1:2002"]
     assert cuda_lib.fn("config_from_properties")(b"/nonexistent/x.properties", C.byref(cfg)) == abi.GPX_EIO
-    # the reference's own loopback config parses (tests/loopback_1_group) when the tree is present
-    ref = "/root/reference/tests/loopback_1_group/gigapaxos.properties"
-    if os.path.exists(ref):
-        assert cuda_lib.fn("config_from_properties")(ref.encode(), C.byref(cfg)) == 0
-        assert cuda_lib.fn("properties_actives")(buf, C.c_size_t(1024)) == 0
-        assert len(buf.value.decode().splitlines()) == 3
+    # the reference's own loopback config (its tests/loopback_1_group/gigapaxos.properties, stored verbatim) parses
+    ref = os.path.join(ROOT, "tests", "golden", "loopback_1_group.gigapaxos.properties")
+    assert cuda_lib.fn("config_from_properties")(ref.encode(), C.byref(cfg)) == 0
+    assert cuda_lib.fn("properties_actives")(buf, C.c_size_t(1024)) == 0
+    assert buf.value.decode().splitlines() == ["100=127.0.0.1:2000", "101=127.0.0.1:2001", "102=127.0.0.1:2002"]
 
 
 def test_java_helpers_in_product_library(cuda_lib):

@@ -525,3 +525,77 @@ def test_create_and_kill_respect_the_pause_table(oracle_lib):
     assert int(rows[0]["acc_slot"]) == 2  # the restored row, not a fresh one
     assert pm.pause("p0") and pm.kill("p0") and not pm.isPaused("p0")
     assert pm.propose("p0", b"y") is None  # gone for good
+
+
+
+def drive_failover_after_wrap(lib, overwritten):
+    """40 groups decide rounds until every lane's 64 KiB log ring has wrapped twice; then the last ACCEPT of groups
+    0..9 reaches only lanes 0 and 1 and is never decided; when `overwritten`, the other groups decide rounds for more
+    than one lap after it.  The next node then runs for coordinator of groups 0..9 (one batch per old coordinator):
+    the carried-over requests' bodies are in the acceptors' rings as long as the ring has not lapped them.  Returns
+    (manager, names, the ten request bodies, the takeover as a callable)."""
+    from helpers import group_descs, make_requests
+    ring = 1 << 16
+    eng = Engine(lib, make_config(lib, max_groups=64, max_batch_recs=4096, max_batch_payload=1 << 20,
+                                  log_ring_bytes=ring))
+    pm = PaxosManager(eng, [HashChainApp() for _ in NODES], NODES, device_phase1b=lib.has("handle_prepare_replies"))
+    names = [f"TESTPaxosApp{i}" for i in range(40)]
+    assert pm.createPaxosInstanceBatch({n: None for n in names}, NODES)
+    r = 0
+    while min(eng.log_head(l) for l in range(3)) < 2 * ring:
+        for n in names:
+            pm.propose(n, b"%s:%d" % (n.encode(), r))
+        pm.run_round()
+        r += 1
+    gids = np.array([pm.instances[n].gid for n in names[:10]], dtype=np.uint32)
+    coord = np.array([NODES.index(int(x)) for x in eng.dump_rows(gids, 0)["acc_bcoord"]])
+    reqs, pay = make_requests(gids, payload_len=9, seed=5)
+    reqs["flags"] = coord << 8
+    reqs["entry_node"] = np.array(NODES)[coord]
+    acc, blob, _ = eng.propose(reqs, pay)
+    acc["dst_mask"] = 0b011
+    eng.handle_accepts(acc, blob)
+    bodies = [bytes(pay[int(o): int(o) + 9]) for o in reqs["payload_off"]]
+    if overwritten:
+        h0 = [eng.log_head(l) for l in range(3)]
+        while min(eng.log_head(l) - h0[l] for l in range(3)) <= ring:
+            for n in names[10:]:
+                pm.propose(n, b"%s:%d" % (n.encode(), r))
+            pm.run_round()
+            r += 1
+
+    def takeover():
+        for c in range(3):
+            won = pm.runForCoordinators([names[i] for i in range(10) if coord[i] == c], (c + 1) % 3)
+            assert all(won.values())
+        pm.run_round()
+    return pm, names, bodies, takeover
+
+
+@pytest.mark.parametrize("overwritten", [False, True])
+def test_failover_after_the_ring_wrapped_cpu(oracle_lib, overwritten):
+    pm, names, bodies, takeover = drive_failover_after_wrap(oracle_lib, overwritten)
+    if overwritten:
+        with pytest.raises(abi.GpxError, match="overwritten"):
+            takeover()
+        return
+    takeover()
+    for n, b in zip(names, bodies):  # the carried-over request executed with its own body on every replica
+        assert all(a.state[n][: len(b)] == b for a in pm.apps)
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("overwritten", [False, True])
+def test_failover_after_the_ring_wrapped_gpu(cuda_lib, oracle_lib, overwritten):
+    (g, names, bodies, tg), (o, _, _, to) = drive_failover_after_wrap(cuda_lib, overwritten), \
+        drive_failover_after_wrap(oracle_lib, overwritten)
+    if overwritten:
+        for t in (tg, to):
+            with pytest.raises(abi.GpxError, match="overwritten"):
+                t()
+        return
+    tg()
+    to()
+    for n, b in zip(names, bodies):
+        assert all(a.state[n][: len(b)] == b for a in g.apps)
+    assert all(a.state == o.apps[0].state and a.seqnum == o.apps[0].seqnum for a in g.apps)
