@@ -23,6 +23,7 @@
 #include <stdint.h>
 
 #include "gpx.h"
+#include "gpx_logseg.cuh"
 
 #define GPX_AUX_STATE(a) ((a) & 0xffu)
 #define GPX_AUX_PRESENT(a) (((a) >> 8) & 0xffu)

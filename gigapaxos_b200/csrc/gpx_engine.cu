@@ -41,6 +41,14 @@ static int fail(int code, const std::string& msg) {
 
 static inline uint32_t cdiv(uint64_t a, uint32_t b) { return (uint32_t)((a + b - 1) / b); }
 
+/* where a launch helper counts and appends: the engine's scratch (gpx_engine::sink()) or a device-resident call's */
+struct Sink {
+  RoundCtl* ctl;
+  gpx_accept_rec* accepts;
+  gpx_exec_rec* extra;
+  uint32_t extra_cap;
+};
+
 struct gpx_engine {
   gpx_config cfg;
   DevState S;
@@ -110,7 +118,6 @@ struct gpx_engine {
   /* timing */
   int n_sms = 148;
   bool timing = false;
-  bool compact_fused = false; /* round_on_stream(fused = false): k_propose + k_act instead of the four phase kernels */
   cudaEvent_t ev[5];
   gpx_kernel_times kt;
 
@@ -122,6 +129,11 @@ struct gpx_engine {
     allocs.push_back(q);
     *p = (T*)q;
     return GPX_OK;
+  }
+  Sink sink() const { return {d_ctl, d_accepts, d_extra, extra_cap}; }
+  /* a device-resident call: the caller's control block and, when given, the caller's extra EXEC queue */
+  Sink sink(gpx_dev_ctl* ctl, gpx_exec_rec* extra = nullptr, uint32_t cap = 0) const {
+    return {reinterpret_cast<RoundCtl*>(ctl), d_accepts, extra ? extra : d_extra, extra ? cap : extra_cap};
   }
   int ensure_misc(size_t bytes) {
     if (bytes <= misc_bytes) return GPX_OK;
@@ -515,22 +527,21 @@ int gpx_patch(gpx_engine* e, uint32_t n, const gpx_patch_rec* p) {
   return GPX_OK;
 }
 
-static void log_advance(gpx_engine* e, uint64_t reserved, bool exact);
 /* every launch that appends to the log reads log_pos[lp] and writes log_pos[lp ^ 1]: flip after the launch */
 static inline void log_flip(gpx_engine* e) { e->S.lp ^= 1u; }
 
 /* ---- kernel launch helpers (device pointers) ------------------------------------- */
-static int launch_propose(gpx_engine* e, const gpx_request_rec* d_reqs, const uint8_t* d_payload,
+static int launch_propose(gpx_engine* e, const Sink& sk, const gpx_request_rec* d_reqs, const uint8_t* d_payload,
                           uint64_t payload_al, uint32_t n, int32_t* d_status, cudaStream_t st) {
   ProposeArgs A;
   A.reqs = d_reqs;
   A.n = n;
   A.payload_bytes_al = payload_al;
-  A.accepts = e->d_accepts;
+  A.accepts = sk.accepts;
   A.status = d_status;
   A.copy_tab = e->d_copy_tab;
   A.copy_dst = e->d_copy_dst;
-  A.ctl = e->d_ctl;
+  A.ctl = sk.ctl;
   k_propose<<<cdiv(n, GPX_BLOCK), GPX_BLOCK, 0, st>>>(e->S, A);
   k_build_blobs<<<cdiv(n, GPX_BLOCK), GPX_BLOCK, 0, st>>>(A, d_payload, e->d_blob1);
   CK(cudaGetLastError());
@@ -550,7 +561,7 @@ static int launch_propose(gpx_engine* e, const gpx_request_rec* d_reqs, const ui
     default: KERNEL<8><<<grid, GPX_BLOCK, 0, st>>>(__VA_ARGS__); break;                \
   }
 
-static int launch_accept(gpx_engine* e, bool fused, const gpx_accept_rec* d_recs, const uint32_t* n_ptr,
+static int launch_accept(gpx_engine* e, const Sink& sk, bool fused, const gpx_accept_rec* d_recs, const uint32_t* n_ptr,
                          uint32_t n_max, const uint8_t* blob0, uint64_t blob0_bytes, const uint8_t* blob1,
                          uint64_t blob1_bytes, const unsigned long long* blob1_used_ptr,
                          gpx_accept_reply_rec* d_replies, gpx_decision_rec* d_dec, gpx_exec_rec* d_exec,
@@ -568,15 +579,10 @@ static int launch_accept(gpx_engine* e, bool fused, const gpx_accept_rec* d_recs
   A.decisions = d_dec;
   A.out_mask = e->d_out_mask;
   A.exec = d_exec;
-  A.extra = e->d_extra;
-  A.extra_cap = e->extra_cap;
-  A.n_extra = &e->d_ctl->n_extra;
+  A.extra = sk.extra;
+  A.extra_cap = sk.extra_cap;
+  A.n_extra = &sk.ctl->n_extra;
   const uint32_t grid = cdiv(n_max, GPX_BLOCK);
-  { /* host mirror of the ring heads: the kernels' own arithmetic (k_accept: one segment; k_act: two, back to back) */
-    const unsigned long long pay_rel = 64ull + (unsigned long long)n_max * 48ull;
-    const unsigned long long res_a = (pay_rel + blob0_bytes + blob1_bytes + 31ull) & ~31ull;
-    log_advance(e, fused ? res_a + 64ull + (unsigned long long)n_max * 32ull : res_a, blob1_used_ptr == nullptr);
-  }
   if (fused) {
     GPX_DISPATCH_L(e->cfg.n_lanes, k_act, grid, st, e->S, A);
   } else {
@@ -587,15 +593,15 @@ static int launch_accept(gpx_engine* e, bool fused, const gpx_accept_rec* d_recs
   return GPX_OK;
 }
 
-static int launch_tally(gpx_engine* e, const gpx_accept_reply_rec* d_replies, const uint32_t* n_ptr, uint32_t mult,
-                        uint32_t n_max, gpx_decision_rec* d_dec, cudaStream_t st) {
+static int launch_tally(gpx_engine* e, const Sink& sk, const gpx_accept_reply_rec* d_replies, const uint32_t* n_ptr,
+                        uint32_t mult, uint32_t n_max, gpx_decision_rec* d_dec, cudaStream_t st) {
   TallyArgs A;
   A.replies = d_replies;
   A.n_ptr = n_ptr;
   A.mult = mult;
   A.n_max = n_max;
   A.decisions = d_dec;
-  A.n_decisions = &e->d_ctl->n_decisions;
+  A.n_decisions = &sk.ctl->n_decisions;
   if (mult > 1 && mult == e->cfg.n_lanes) { /* [ACCEPT][lane] layout of the phase pipeline: one thread per slot */
     GPX_DISPATCH_L(mult, k_tally_slots, cdiv(n_max / mult, GPX_BLOCK), st, e->S, A);
   } else
@@ -604,17 +610,16 @@ static int launch_tally(gpx_engine* e, const gpx_accept_reply_rec* d_replies, co
   return GPX_OK;
 }
 
-static int launch_commit(gpx_engine* e, const gpx_decision_rec* d_dec, const uint32_t* n_ptr, uint32_t n_max,
-                         gpx_exec_rec* d_exec, cudaStream_t st) {
+static int launch_commit(gpx_engine* e, const Sink& sk, const gpx_decision_rec* d_dec, const uint32_t* n_ptr,
+                         uint32_t n_max, gpx_exec_rec* d_exec, cudaStream_t st) {
   CommitArgs A;
   A.decisions = d_dec;
   A.n_ptr = n_ptr;
   A.n_max = n_max;
   A.exec = d_exec;
-  A.extra = e->d_extra;
-  A.extra_cap = e->extra_cap;
-  A.n_extra = &e->d_ctl->n_extra;
-  log_advance(e, 64ull + (unsigned long long)n_max * 32ull, true);
+  A.extra = sk.extra;
+  A.extra_cap = sk.extra_cap;
+  A.n_extra = &sk.ctl->n_extra;
   GPX_DISPATCH_L(e->cfg.n_lanes, k_commit, cdiv(n_max, GPX_BLOCK), st, e->S, A);
   log_flip(e);
   CK(cudaGetLastError());
@@ -643,6 +648,10 @@ static void launch_round_t(uint32_t grid, cudaStream_t st, const DevState& S, co
     cudaLaunchKernelEx(&cfg, k_round_slow<L, LP>, S, RA);
   }
 }
+}
+/* payload-area bytes a round of n requests reserves for the blobs it constructs for batched slots */
+static uint64_t blob1_res(const gpx_engine* e, uint32_t n, uint64_t pal) {
+  return e->cfg.batching_enabled ? std::min<uint64_t>(e->blob1_cap, 16ull * n + pal) : 0;
 }
 static int launch_round(gpx_engine* e, const gpx_request_rec* d_reqs, const uint8_t* d_payload, uint64_t pal,
                         uint32_t n, int32_t* d_status, gpx_exec_rec* d_exec, cudaStream_t st,
@@ -689,13 +698,12 @@ static int launch_round(gpx_engine* e, const gpx_request_rec* d_reqs, const uint
   RA.todo_end = e->d_todo + e->cfg.max_batch_recs;
   RA.mark = e->d_mark;
   RA.n_todo = &d_ctl->n_todo;
-  RA.blob1_res = e->cfg.batching_enabled ? std::min<uint64_t>(e->blob1_cap, 16ull * n + pal) : 0;
+  RA.blob1_res = blob1_res(e, n, pal);
   RA.A.blob1_bytes = RA.blob1_res;
   RA.pay_bytes = pal + RA.blob1_res;
-  RA.pay_rel = 64u + n * 48u;
-  RA.res_a = ((unsigned long long)RA.pay_rel + RA.pay_bytes + 31ull) & ~31ull;
-  RA.res_d = 64ull + (unsigned long long)n * 32ull;
-  log_advance(e, RA.res_a + RA.res_d, true);
+  RA.pay_rel = (uint32_t)seg_pay_rel(n);
+  RA.res_a = seg_accept_bytes(n, RA.pay_bytes);
+  RA.res_d = seg_decision_bytes(n);
   const uint32_t L = e->cfg.n_lanes;
   const uint32_t teams_per_block = (GPX_RBLOCK / 32u) * (32u / L); /* teams of L adjacent lanes */
   const uint32_t grid = cdiv((uint64_t)n, teams_per_block);
@@ -718,40 +726,68 @@ static int launch_round(gpx_engine* e, const gpx_request_rec* d_reqs, const uint
 }
 
 /* ---- log ring bookkeeping on the host ------------------------------------------------------------------ */
-static int log_resync(gpx_engine* e) { /* the true heads, after everything enqueued so far */
-  if (e->head_exact) return GPX_OK;
+/* What one API call appends to every lane: up to two reservations, in launch order (an unused one is 0 bytes).  A
+ * reservation is what one seg_base takes on the device: a segment, or a pair of segments laid out back to back (k_act,
+ * k_round).  exact = false: an ACCEPT segment's payload area is a count the kernels read on the device, and its size
+ * here is an upper bound. */
+struct LogSegs {
+  uint64_t bytes[2];
+  bool exact;
+};
+static LogSegs one_seg(uint64_t bytes) { return {{bytes, 0}, true}; }
+
+enum class RoundForm {
+  FUSED,   /* k_round (+ k_round_slow): outputs indexed by request */
+  COMPACT, /* k_propose + k_act: one record, log image and EXEC row per ACCEPT */
+  PHASES,  /* k_propose, k_accept, k_tally, k_commit */
+};
+static LogSegs round_segs(const gpx_engine* e, RoundForm form, uint32_t n, uint64_t payload_bytes) {
+  const uint64_t pal = (payload_bytes + 15) & ~15ull;
+  const uint64_t a = seg_accept_bytes(n, pal + blob1_res(e, n, pal)), d = seg_decision_bytes(n);
+  if (form == RoundForm::PHASES) return {{a, d}, false};
+  return {{a + d, 0}, form == RoundForm::FUSED};
+}
+
+/* the heads the next logging launch will start from, after everything enqueued so far on any stream */
+static int read_device_heads(gpx_engine* e, uint64_t out[GPX_MAX_LANES]) {
   CK(cudaDeviceSynchronize());
-  unsigned long long pos[2 * GPX_MAX_LANES]; /* the copy the next launch will read: {head, seq} per lane */
+  unsigned long long pos[2 * GPX_MAX_LANES]; /* {head, seq} per lane */
   CK(cudaMemcpy(pos, e->S.log_pos + (size_t)e->S.lp * 2 * GPX_MAX_LANES, sizeof pos, cudaMemcpyDeviceToHost));
-  for (uint32_t l = 0; l < e->cfg.n_lanes; l++) e->h_head[l] = pos[2 * l];
+  for (uint32_t l = 0; l < e->cfg.n_lanes; l++) out[l] = pos[2 * l];
+  return GPX_OK;
+}
+static int log_resync(gpx_engine* e) {
+  if (e->head_exact) return GPX_OK;
+  int rc = read_device_heads(e, e->h_head);
+  if (rc) return rc;
   e->head_exact = true;
   return GPX_OK;
 }
-/* what seg_base + the publishing block do on the device, on the mirror: one segment (or one pair of segments laid out
- * back to back) of `reserved` bytes is appended to every lane; `exact` = the host knows `reserved` */
-static void log_advance(gpx_engine* e, uint64_t reserved, bool exact) {
-  if (!e->cfg.log_ring_bytes) return;
-  if (!exact) e->head_exact = false;
+/* what seg_base + the publishing block do on the device, on the mirror */
+static void log_advance(gpx_engine* e, const LogSegs& s) {
+  if (!s.exact) e->head_exact = false;
   if (!e->head_exact) return;
   const uint64_t cap = e->cfg.log_ring_bytes;
-  for (uint32_t l = 0; l < e->cfg.n_lanes; l++) {
-    uint64_t h = e->h_head[l];
-    const uint64_t pos = h & (cap - 1);
-    if (pos + reserved > cap) h += cap - pos;
-    e->h_head[l] = h + reserved;
-  }
+  for (const uint64_t reserved : s.bytes)
+    for (uint32_t l = 0; l < e->cfg.n_lanes; l++) {
+      uint64_t h = e->h_head[l];
+      const uint64_t pos = h & (cap - 1);
+      if (pos + reserved > cap) h += cap - pos;
+      e->h_head[l] = h + reserved;
+    }
 }
-/* `reserved` = upper bound of what one API call appends per lane.  With log_backpressure the call is refused
- * (GPX_EAGAIN, nothing has happened yet) when it could overwrite bytes that were not released (gpx_log_release):
- * AbstractPaxosLogger.logAndMessage :157 logs THEN messages -- an ACCEPT_REPLY may only leave once its ACCEPT is
- * durable, so the journal must have been drained before the ring position is reused. */
-static int ring_fits(gpx_engine* e, uint64_t reserved) {
-  if (reserved > e->cfg.log_ring_bytes) return fail(GPX_ERANGE, "batch does not fit the log ring; raise log_ring_bytes");
+/* With log_backpressure the call is refused (GPX_EAGAIN, nothing has happened yet) when it could overwrite bytes that
+ * were not released (gpx_log_release): AbstractPaxosLogger.logAndMessage :157 logs THEN messages -- an ACCEPT_REPLY may
+ * only leave once its ACCEPT is durable, so the journal must have been drained before the ring position is reused. */
+static int ring_fits(gpx_engine* e, const LogSegs& s) {
+  const uint64_t total = s.bytes[0] + s.bytes[1];
+  if (total > e->cfg.log_ring_bytes) return fail(GPX_ERANGE, "batch does not fit the log ring; raise log_ring_bytes");
   if (e->cfg.log_backpressure) {
     int rc = log_resync(e);
     if (rc) return rc;
-    for (uint32_t l = 0; l < e->cfg.n_lanes; l++) /* 2 x: every segment of the call may first skip to the ring start */
-      if (e->h_head[l] - e->log_tail[l] + 2 * reserved > e->cfg.log_ring_bytes)
+    for (uint32_t l = 0; l < e->cfg.n_lanes; l++) /* 2 x: a reservation may first skip to the ring start, and that skip
+                                                    * is shorter than the reservation */
+      if (e->h_head[l] - e->log_tail[l] + 2 * total > e->cfg.log_ring_bytes)
         return fail(GPX_EAGAIN, "log ring full: drain it (gpx_log_drain_async) and release the drained bytes (gpx_log_release)");
   }
   return GPX_OK;
@@ -764,6 +800,17 @@ static int check_batch(gpx_engine* e, uint32_t n, uint64_t payload_bytes) {
 static int fetch_ctl(gpx_engine* e, const RoundCtl* src = nullptr) {
   CK(cudaMemcpyAsync(e->h_ctl, src ? src : e->d_ctl, sizeof(RoundCtl), cudaMemcpyDeviceToHost, e->stream));
   CK(cudaStreamSynchronize(e->stream));
+  return GPX_OK;
+}
+/* the engine's extra EXEC queue, as counted in h_ctl, to the caller: at most cap records; *n_extra = the whole count */
+static int copy_extra_out(gpx_engine* e, gpx_exec_rec* dst, uint32_t cap, uint32_t* n_extra) {
+  const uint32_t nx = e->h_ctl->n_extra;
+  if (n_extra) *n_extra = nx;
+  const uint32_t cp = std::min(std::min(nx, cap), e->extra_cap);
+  if (cp && dst) {
+    CK(cudaMemcpyAsync(dst, e->d_extra, cp * sizeof(gpx_exec_rec), cudaMemcpyDeviceToHost, e->stream));
+    CK(cudaStreamSynchronize(e->stream));
+  }
   return GPX_OK;
 }
 
@@ -783,7 +830,7 @@ int gpx_propose(gpx_engine* e, uint32_t n, const gpx_request_rec* reqs, const ui
   CK(cudaMemsetAsync(e->d_ctl, 0, sizeof(RoundCtl), st));
   CK(cudaMemcpyAsync(e->d_reqs, reqs, n * sizeof(gpx_request_rec), cudaMemcpyHostToDevice, st));
   if (payload_bytes) CK(cudaMemcpyAsync(e->d_payload, payload, payload_bytes, cudaMemcpyHostToDevice, st));
-  rc = launch_propose(e, e->d_reqs, e->d_payload, pal, n, e->d_status, st);
+  rc = launch_propose(e, e->sink(), e->d_reqs, e->d_payload, pal, n, e->d_status, st);
   if (rc) return rc;
   rc = fetch_ctl(e);
   if (rc) return rc;
@@ -813,28 +860,23 @@ int gpx_handle_accepts(gpx_engine* e, uint32_t n, const gpx_accept_rec* accepts,
   if (blob_bytes & 15) return fail(GPX_EINVAL, "blob_bytes must be a multiple of 16");
   if (n > e->cfg.max_batch_recs) return fail(GPX_ERANGE, "n > max_batch_recs");
   if (blob_bytes > e->blob1_cap) return fail(GPX_ERANGE, "blob too large");
-  int rc = ring_fits(e, 96ull + 48ull * n + blob_bytes);
+  const LogSegs segs = one_seg(seg_accept_bytes(n, blob_bytes));
+  int rc = ring_fits(e, segs);
   if (rc) return rc;
   cudaStream_t st = e->stream;
   const uint32_t L = e->cfg.n_lanes;
   CK(cudaMemsetAsync(e->d_ctl, 0, sizeof(RoundCtl), st));
   CK(cudaMemcpyAsync(e->d_accepts, accepts, n * sizeof(gpx_accept_rec), cudaMemcpyHostToDevice, st));
   if (blob_bytes) CK(cudaMemcpyAsync(e->d_blob1, blob, blob_bytes, cudaMemcpyHostToDevice, st));
-  rc = launch_accept(e, false, e->d_accepts, nullptr, n, e->d_blob1, blob_bytes, nullptr, 0, nullptr, e->d_replies,
-                     nullptr, nullptr, st);
+  log_advance(e, segs);
+  rc = launch_accept(e, e->sink(), false, e->d_accepts, nullptr, n, e->d_blob1, blob_bytes, nullptr, 0, nullptr,
+                     e->d_replies, nullptr, nullptr, st);
   if (rc) return rc;
   CK(cudaMemcpyAsync(out_replies, e->d_replies, (size_t)n * L * sizeof(gpx_accept_reply_rec), cudaMemcpyDeviceToHost,
                      st));
   rc = fetch_ctl(e);
   if (rc) return rc;
-  uint32_t nx = e->h_ctl->n_extra;
-  if (n_extra) *n_extra = nx;
-  uint32_t cp = std::min(std::min(nx, extra_cap), e->extra_cap);
-  if (cp && out_extra_exec) {
-    CK(cudaMemcpyAsync(out_extra_exec, e->d_extra, cp * sizeof(gpx_exec_rec), cudaMemcpyDeviceToHost, st));
-    CK(cudaStreamSynchronize(st));
-  }
-  return GPX_OK;
+  return copy_extra_out(e, out_extra_exec, extra_cap, n_extra);
 }
 
 int gpx_handle_accept_replies(gpx_engine* e, uint32_t n, const gpx_accept_reply_rec* replies,
@@ -847,7 +889,7 @@ int gpx_handle_accept_replies(gpx_engine* e, uint32_t n, const gpx_accept_reply_
   cudaStream_t st = e->stream;
   CK(cudaMemsetAsync(e->d_ctl, 0, sizeof(RoundCtl), st));
   CK(cudaMemcpyAsync(e->d_replies, replies, n * sizeof(gpx_accept_reply_rec), cudaMemcpyHostToDevice, st));
-  int rc = launch_tally(e, e->d_replies, nullptr, 1, n, e->d_decisions, st);
+  int rc = launch_tally(e, e->sink(), e->d_replies, nullptr, 1, n, e->d_decisions, st);
   if (rc) return rc;
   rc = fetch_ctl(e);
   if (rc) return rc;
@@ -867,25 +909,20 @@ int gpx_handle_decisions(gpx_engine* e, uint32_t n, const gpx_decision_rec* deci
   if (n == 0) return GPX_OK;
   if (!decisions || !out_exec) return fail(GPX_EINVAL, "null argument");
   if (n > (uint64_t)e->cfg.max_batch_recs) return fail(GPX_ERANGE, "n > max_batch_recs");
-  int rc = ring_fits(e, 64ull + 32ull * n);
+  const LogSegs segs = one_seg(seg_decision_bytes(n));
+  int rc = ring_fits(e, segs);
   if (rc) return rc;
   cudaStream_t st = e->stream;
   const uint32_t L = e->cfg.n_lanes;
   CK(cudaMemsetAsync(e->d_ctl, 0, sizeof(RoundCtl), st));
   CK(cudaMemcpyAsync(e->d_decisions, decisions, n * sizeof(gpx_decision_rec), cudaMemcpyHostToDevice, st));
-  rc = launch_commit(e, e->d_decisions, nullptr, n, e->d_exec, st);
+  log_advance(e, segs);
+  rc = launch_commit(e, e->sink(), e->d_decisions, nullptr, n, e->d_exec, st);
   if (rc) return rc;
   CK(cudaMemcpyAsync(out_exec, e->d_exec, (size_t)n * L * sizeof(gpx_exec_rec), cudaMemcpyDeviceToHost, st));
   rc = fetch_ctl(e);
   if (rc) return rc;
-  uint32_t nx = e->h_ctl->n_extra;
-  if (n_extra) *n_extra = nx;
-  uint32_t cp = std::min(std::min(nx, extra_cap), e->extra_cap);
-  if (cp && out_extra_exec) {
-    CK(cudaMemcpyAsync(out_extra_exec, e->d_extra, cp * sizeof(gpx_exec_rec), cudaMemcpyDeviceToHost, st));
-    CK(cudaStreamSynchronize(st));
-  }
-  return GPX_OK;
+  return copy_extra_out(e, out_extra_exec, extra_cap, n_extra);
 }
 
 /* phase 1a at the acceptors: PISM.handlePrepare for a batch of PREPAREs, host buffers */
@@ -894,7 +931,8 @@ int gpx_handle_prepares(gpx_engine* e, uint32_t n, const gpx_pvalue_hdr* prepare
   if (n == 0) return GPX_OK;
   if (!prepares || !out_replies) return fail(GPX_EINVAL, "null argument");
   if (n > e->cfg.max_batch_recs) return fail(GPX_ERANGE, "n > max_batch_recs");
-  int rc = ring_fits(e, 64ull + 32ull * n);
+  const LogSegs segs = one_seg(seg_decision_bytes(n));
+  int rc = ring_fits(e, segs);
   if (rc) return rc;
   const uint32_t L = e->cfg.n_lanes;
   const size_t out_bytes = (size_t)n * L * sizeof(gpx_prepare_reply_rec);
@@ -906,7 +944,7 @@ int gpx_handle_prepares(gpx_engine* e, uint32_t n, const gpx_pvalue_hdr* prepare
   A.recs = e->d_decisions;
   A.n = n;
   A.replies = (gpx_prepare_reply_rec*)e->d_misc;
-  log_advance(e, 64ull + 32ull * n, true);
+  log_advance(e, segs);
   GPX_DISPATCH_L(L, k_prepare, cdiv(n, GPX_BLOCK), st, e->S, A);
   log_flip(e);
   CK(cudaGetLastError());
@@ -966,15 +1004,17 @@ int gpx_handle_accepts_fused(gpx_engine* e, uint32_t n, const gpx_accept_rec* ac
   if (blob_bytes & 15) return fail(GPX_EINVAL, "blob_bytes must be a multiple of 16");
   if (n > e->cfg.max_batch_recs) return fail(GPX_ERANGE, "n > max_batch_recs");
   if (blob_bytes > e->blob1_cap) return fail(GPX_ERANGE, "blob too large");
-  int rc = ring_fits(e, 160ull + 80ull * n + blob_bytes);
+  const LogSegs segs = one_seg(seg_accept_bytes(n, blob_bytes) + seg_decision_bytes(n));
+  int rc = ring_fits(e, segs);
   if (rc) return rc;
   cudaStream_t st = e->stream;
   const uint32_t L = e->cfg.n_lanes;
   CK(cudaMemsetAsync(e->d_ctl, 0, sizeof(RoundCtl), st));
   CK(cudaMemcpyAsync(e->d_accepts, accepts, n * sizeof(gpx_accept_rec), cudaMemcpyHostToDevice, st));
   if (blob_bytes) CK(cudaMemcpyAsync(e->d_blob1, blob, blob_bytes, cudaMemcpyHostToDevice, st));
-  rc = launch_accept(e, true, e->d_accepts, nullptr, n, e->d_blob1, blob_bytes, nullptr, 0, nullptr, e->d_replies,
-                     e->d_decisions, e->d_exec, st);
+  log_advance(e, segs);
+  rc = launch_accept(e, e->sink(), true, e->d_accepts, nullptr, n, e->d_blob1, blob_bytes, nullptr, 0, nullptr,
+                     e->d_replies, e->d_decisions, e->d_exec, st);
   if (rc) return rc;
   /* replies consumed by a local coordinator never reach HBM: out_mask says which reply slots were written */
   e->h_out_mask.resize(n);
@@ -998,25 +1038,19 @@ int gpx_handle_accepts_fused(gpx_engine* e, uint32_t n, const gpx_accept_rec* ac
         r.slot = accepts[i].h.slot;
         r.who = GPX_WHO(0xffu, 0xffu, GPX_F_VOID);
       }
-  uint32_t nx = e->h_ctl->n_extra;
-  if (n_extra) *n_extra = nx;
-  uint32_t cp = std::min(std::min(nx, extra_cap), e->extra_cap);
-  if (cp && out_extra_exec) {
-    CK(cudaMemcpyAsync(out_extra_exec, e->d_extra, cp * sizeof(gpx_exec_rec), cudaMemcpyDeviceToHost, st));
-    CK(cudaStreamSynchronize(st));
-  }
-  return GPX_OK;
+  return copy_extra_out(e, out_extra_exec, extra_cap, n_extra);
 }
 
-/* one round on device pointers.  fused: k_propose -> k_act (replies, decisions and rows stay in registers);
- * phases: k_propose -> k_accept -> k_tally -> k_commit (inter-replica records go through HBM) */
-static int round_on_stream(gpx_engine* e, bool fused, const gpx_request_rec* d_reqs, const uint8_t* d_payload,
-                           uint64_t payload_bytes, uint32_t n, int32_t* d_status, gpx_exec_rec* d_exec,
-                           cudaStream_t st) {
+/* one round on device pointers; `segs` = round_segs(e, form, ...), already admitted by ring_fits */
+static int round_on_stream(gpx_engine* e, RoundForm form, const LogSegs& segs, const gpx_request_rec* d_reqs,
+                           const uint8_t* d_payload, uint64_t payload_bytes, uint32_t n, int32_t* d_status,
+                           gpx_exec_rec* d_exec, cudaStream_t st) {
   const uint64_t pal = (payload_bytes + 15) & ~15ull;
   const uint32_t L = e->cfg.n_lanes;
   const bool tm = e->timing;
+  const bool fused = form == RoundForm::FUSED, compact = form == RoundForm::COMPACT;
   if (!fused) CK(cudaMemsetAsync(e->d_ctl, 0, sizeof(RoundCtl), st)); /* the fused kernels keep their own block zero */
+  log_advance(e, segs);
   if (tm) cudaEventRecord(e->ev[0], st);
   if (fused) { /* the whole round is ONE kernel */
     int rc1 = launch_round(e, d_reqs, d_payload, pal, n, d_status, d_exec, st);
@@ -1031,21 +1065,22 @@ static int round_on_stream(gpx_engine* e, bool fused, const gpx_request_rec* d_r
     }
     return GPX_OK;
   }
-  int rc = launch_propose(e, d_reqs, d_payload, pal, n, d_status, st);
+  const Sink sk = e->sink();
+  int rc = launch_propose(e, sk, d_reqs, d_payload, pal, n, d_status, st);
   if (rc) return rc;
   if (tm) cudaEventRecord(e->ev[1], st);
   /* the ACCEPT segment mirrors the payload arena plus the constructed blobs actually used */
-  rc = launch_accept(e, e->compact_fused, e->d_accepts, &e->d_ctl->n_accepts, n, d_payload, pal, e->d_blob1, 0,
-                     &e->d_ctl->blob1_used, e->d_replies, e->d_decisions, d_exec, st);
+  rc = launch_accept(e, sk, compact, sk.accepts, &sk.ctl->n_accepts, n, d_payload, pal, e->d_blob1, 0,
+                     &sk.ctl->blob1_used, e->d_replies, e->d_decisions, d_exec, st);
   if (rc) return rc;
   if (tm) cudaEventRecord(e->ev[2], st);
-  if (!e->compact_fused) {
-    rc = launch_tally(e, e->d_replies, &e->d_ctl->n_accepts, L, n * L, e->d_decisions, st);
+  if (!compact) {
+    rc = launch_tally(e, sk, e->d_replies, &sk.ctl->n_accepts, L, n * L, e->d_decisions, st);
     if (rc) return rc;
   }
-  if (tm) cudaEventRecord(e->ev[3], st);
-  if (!e->compact_fused) {
-    rc = launch_commit(e, e->d_decisions, &e->d_ctl->n_decisions, n, d_exec, st);
+  if (tm) cudaEventRecord(e->ev[3], st); /* compact: the tally and commit intervals are empty */
+  if (!compact) {
+    rc = launch_commit(e, sk, e->d_decisions, &sk.ctl->n_decisions, n, d_exec, st);
     if (rc) return rc;
   }
   if (tm) {
@@ -1072,7 +1107,7 @@ int gpx_set_round_mode(gpx_engine* e, int mode) {
   return GPX_OK;
 }
 
-static int round_host(gpx_engine* e, bool fused, uint32_t n, const gpx_request_rec* reqs, const uint8_t* payload,
+static int round_host(gpx_engine* e, RoundForm form, uint32_t n, const gpx_request_rec* reqs, const uint8_t* payload,
                       uint64_t payload_bytes, int32_t* status, gpx_exec_rec* out_exec, uint32_t* n_exec_slots,
                       gpx_exec_rec* out_extra_exec, uint32_t extra_cap, uint32_t* n_extra) {
   if (!e || !n_exec_slots) return fail(GPX_EINVAL, "null argument");
@@ -1082,104 +1117,67 @@ static int round_host(gpx_engine* e, bool fused, uint32_t n, const gpx_request_r
   if (!reqs || !status || !out_exec || (!payload && payload_bytes)) return fail(GPX_EINVAL, "null argument");
   int rc = check_batch(e, n, payload_bytes);
   if (rc) return rc;
-  const uint64_t pal = (payload_bytes + 15) & ~15ull;
-  const uint64_t b1 = e->cfg.batching_enabled ? std::min<uint64_t>(e->blob1_cap, 16ull * n + pal) : 0;
-  rc = ring_fits(e, 192ull + 80ull * n + pal + b1);
+  const LogSegs segs = round_segs(e, form, n, payload_bytes);
+  rc = ring_fits(e, segs);
   if (rc) return rc;
   cudaStream_t st = e->stream;
   const uint32_t L = e->cfg.n_lanes;
   CK(cudaMemcpyAsync(e->d_reqs, reqs, n * sizeof(gpx_request_rec), cudaMemcpyHostToDevice, st));
   if (payload_bytes) CK(cudaMemcpyAsync(e->d_payload, payload, payload_bytes, cudaMemcpyHostToDevice, st));
-  rc = round_on_stream(e, fused, e->d_reqs, e->d_payload, payload_bytes, n, e->d_status, e->d_exec, st);
+  rc = round_on_stream(e, form, segs, e->d_reqs, e->d_payload, payload_bytes, n, e->d_status, e->d_exec, st);
   if (rc) return rc;
   CK(cudaMemcpyAsync(status, e->d_status, n * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
-  rc = fetch_ctl(e, fused ? e->last_ctl : nullptr);
+  rc = fetch_ctl(e, form == RoundForm::FUSED ? e->last_ctl : nullptr);
   if (rc) return rc;
   /* fused: one EXEC row per REQUEST index (VOID where the request carries no ACCEPT); phases: one per DECISION */
-  const uint32_t rows = fused ? n : e->h_ctl->n_decisions;
-  const uint32_t nx = e->h_ctl->n_extra;
+  const uint32_t rows = form == RoundForm::FUSED ? n : e->h_ctl->n_decisions;
   if (rows) CK(cudaMemcpyAsync(out_exec, e->d_exec, (size_t)rows * L * sizeof(gpx_exec_rec), cudaMemcpyDeviceToHost, st));
-  uint32_t cp = std::min(std::min(nx, extra_cap), e->extra_cap);
-  if (cp && out_extra_exec)
-    CK(cudaMemcpyAsync(out_extra_exec, e->d_extra, cp * sizeof(gpx_exec_rec), cudaMemcpyDeviceToHost, st));
+  rc = copy_extra_out(e, out_extra_exec, extra_cap, n_extra);
+  if (rc) return rc;
   CK(cudaStreamSynchronize(st));
   *n_exec_slots = rows * L;
-  if (n_extra) *n_extra = nx;
   return GPX_OK;
 }
 
 int gpx_round(gpx_engine* e, uint32_t n, const gpx_request_rec* reqs, const uint8_t* payload, uint64_t payload_bytes,
               int32_t* status, gpx_exec_rec* out_exec, uint32_t* n_exec_slots, gpx_exec_rec* out_extra_exec,
               uint32_t extra_cap, uint32_t* n_extra) {
-  return round_host(e, true, n, reqs, payload, payload_bytes, status, out_exec, n_exec_slots, out_extra_exec,
-                    extra_cap, n_extra);
+  return round_host(e, RoundForm::FUSED, n, reqs, payload, payload_bytes, status, out_exec, n_exec_slots,
+                    out_extra_exec, extra_cap, n_extra);
 }
 int gpx_round_phases(gpx_engine* e, uint32_t n, const gpx_request_rec* reqs, const uint8_t* payload,
                      uint64_t payload_bytes, int32_t* status, gpx_exec_rec* out_exec, uint32_t* n_exec_slots,
                      gpx_exec_rec* out_extra_exec, uint32_t extra_cap, uint32_t* n_extra) {
-  return round_host(e, false, n, reqs, payload, payload_bytes, status, out_exec, n_exec_slots, out_extra_exec,
-                    extra_cap, n_extra);
+  return round_host(e, RoundForm::PHASES, n, reqs, payload, payload_bytes, status, out_exec, n_exec_slots,
+                    out_extra_exec, extra_cap, n_extra);
 }
 
-int gpx_round_device(gpx_engine* e, const gpx_dev_round_bufs* b, void* stream) {
+static int round_device(gpx_engine* e, RoundForm form, const gpx_dev_round_bufs* b, void* stream) {
   if (!e || !b) return fail(GPX_EINVAL, "null argument");
   if (b->n == 0) return GPX_OK;
   int rc = check_batch(e, b->n, b->payload_bytes);
   if (rc) return rc;
-  return round_on_stream(e, true, b->reqs, b->payload, b->payload_bytes, b->n, b->status, b->exec,
+  const LogSegs segs = round_segs(e, form, b->n, b->payload_bytes);
+  rc = ring_fits(e, segs);
+  if (rc) return rc;
+  return round_on_stream(e, form, segs, b->reqs, b->payload, b->payload_bytes, b->n, b->status, b->exec,
                          stream ? (cudaStream_t)stream : e->stream);
+}
+int gpx_round_device(gpx_engine* e, const gpx_dev_round_bufs* b, void* stream) {
+  return round_device(e, RoundForm::FUSED, b, stream);
 }
 /* k_propose (ACCEPTs compacted at the front: one record, log image and EXEC row per ACCEPT, no per-request holes) +
  * k_act (accept -> tally -> commit per ACCEPT in registers): the form for batches in which most requests share a
  * slot with others (RequestBatcher.java:198-219) */
 int gpx_round_device_compact(gpx_engine* e, const gpx_dev_round_bufs* b, void* stream) {
-  if (!e || !b) return fail(GPX_EINVAL, "null argument");
-  if (b->n == 0) return GPX_OK;
-  int rc = check_batch(e, b->n, b->payload_bytes);
-  if (rc) return rc;
-  e->compact_fused = true;
-  rc = round_on_stream(e, false, b->reqs, b->payload, b->payload_bytes, b->n, b->status, b->exec,
-                       stream ? (cudaStream_t)stream : e->stream);
-  e->compact_fused = false;
-  return rc;
+  return round_device(e, RoundForm::COMPACT, b, stream);
 }
 int gpx_round_device_phases(gpx_engine* e, const gpx_dev_round_bufs* b, void* stream) {
-  if (!e || !b) return fail(GPX_EINVAL, "null argument");
-  if (b->n == 0) return GPX_OK;
-  int rc = check_batch(e, b->n, b->payload_bytes);
-  if (rc) return rc;
-  return round_on_stream(e, false, b->reqs, b->payload, b->payload_bytes, b->n, b->status, b->exec,
-                         stream ? (cudaStream_t)stream : e->stream);
+  return round_device(e, RoundForm::PHASES, b, stream);
 }
 
 /* ---- device-resident phase calls (spread placement) -------------------------------------- */
 static_assert(sizeof(gpx_dev_ctl) == sizeof(RoundCtl), "gpx_dev_ctl mirrors RoundCtl");
-namespace {
-/* the launch helpers count into / append to engine-owned scratch; point them at the caller's buffers for the
- * duration of one call (the engine is single-submitter) */
-struct ScratchSwap {
-  gpx_engine* e;
-  RoundCtl* ctl0;
-  gpx_accept_rec* acc0;
-  gpx_exec_rec* ex0;
-  uint32_t cap0;
-  ScratchSwap(gpx_engine* e_, gpx_dev_ctl* ctl, gpx_accept_rec* acc, gpx_exec_rec* extra, uint32_t extra_cap)
-      : e(e_), ctl0(e_->d_ctl), acc0(e_->d_accepts), ex0(e_->d_extra), cap0(e_->extra_cap) {
-    if (ctl) e->d_ctl = reinterpret_cast<RoundCtl*>(ctl);
-    if (acc) e->d_accepts = acc;
-    if (extra) {
-      e->d_extra = extra;
-      e->extra_cap = extra_cap;
-    }
-  }
-  ~ScratchSwap() {
-    e->d_ctl = ctl0;
-    e->d_accepts = acc0;
-    e->d_extra = ex0;
-    e->extra_cap = cap0;
-  }
-};
-}  // namespace
 
 int gpx_propose_device(gpx_engine* e, const gpx_request_rec* reqs, const uint8_t* payload, uint64_t payload_bytes,
                        uint32_t n, int32_t* status, gpx_accept_rec* out_accepts, gpx_dev_ctl* ctl, void* stream) {
@@ -1188,8 +1186,9 @@ int gpx_propose_device(gpx_engine* e, const gpx_request_rec* reqs, const uint8_t
   if (!reqs || !status || !out_accepts || (!payload && payload_bytes)) return fail(GPX_EINVAL, "null argument");
   int rc = check_batch(e, n, payload_bytes);
   if (rc) return rc;
-  ScratchSwap sw(e, ctl, out_accepts, nullptr, 0);
-  return launch_propose(e, reqs, payload, (payload_bytes + 15) & ~15ull, n, status,
+  Sink sk = e->sink(ctl);
+  sk.accepts = out_accepts;
+  return launch_propose(e, sk, reqs, payload, (payload_bytes + 15) & ~15ull, n, status,
                         stream ? (cudaStream_t)stream : e->stream);
 }
 
@@ -1235,7 +1234,8 @@ int gpx_accepts_device(gpx_engine* e, gpx_accept_rec* recs, uint32_t n, const ui
   if (blob_bytes & 15) return fail(GPX_EINVAL, "blob_bytes must be a multiple of 16");
   if (n_chunks > GPX_ROUTE_ND || (n_chunks && (!chunk_rec_end || !chunk_blob_base))) return fail(GPX_EINVAL, "chunks");
   if (n > e->cfg.max_batch_recs) return fail(GPX_ERANGE, "n > max_batch_recs");
-  int rc = ring_fits(e, 96ull + 48ull * n + blob_bytes);
+  const LogSegs segs = one_seg(seg_accept_bytes(n, blob_bytes));
+  int rc = ring_fits(e, segs);
   if (rc) return rc;
   cudaStream_t st = stream ? (cudaStream_t)stream : e->stream;
   {
@@ -1251,9 +1251,9 @@ int gpx_accepts_device(gpx_engine* e, gpx_accept_rec* recs, uint32_t n, const ui
     }
     k_ingest<<<cdiv(n, GPX_BLOCK), GPX_BLOCK, 0, st>>>(e->S, R);
   }
-  ScratchSwap sw(e, ctl, nullptr, out_extra, out_extra ? extra_cap : 0);
-  return launch_accept(e, false, recs, nullptr, n, blob, blob_bytes, nullptr, 0, nullptr, out_replies, nullptr, nullptr,
-                       st);
+  log_advance(e, segs);
+  return launch_accept(e, e->sink(ctl, out_extra, extra_cap), false, recs, nullptr, n, blob, blob_bytes, nullptr, 0,
+                       nullptr, out_replies, nullptr, nullptr, st);
 }
 
 int gpx_replies_device(gpx_engine* e, const gpx_accept_reply_rec* replies, uint32_t n,
@@ -1261,8 +1261,7 @@ int gpx_replies_device(gpx_engine* e, const gpx_accept_reply_rec* replies, uint3
   if (!e || !ctl) return fail(GPX_EINVAL, "null argument");
   if (n == 0) return GPX_OK;
   if (!replies || !out_decisions) return fail(GPX_EINVAL, "null argument");
-  ScratchSwap sw(e, ctl, nullptr, nullptr, 0);
-  return launch_tally(e, replies, nullptr, 1, n, out_decisions, stream ? (cudaStream_t)stream : e->stream);
+  return launch_tally(e, e->sink(ctl), replies, nullptr, 1, n, out_decisions, stream ? (cudaStream_t)stream : e->stream);
 }
 
 int gpx_decisions_device(gpx_engine* e, gpx_decision_rec* decisions, uint32_t n, gpx_exec_rec* out_exec,
@@ -1271,7 +1270,8 @@ int gpx_decisions_device(gpx_engine* e, gpx_decision_rec* decisions, uint32_t n,
   if (n == 0) return GPX_OK;
   if (!decisions || !out_exec) return fail(GPX_EINVAL, "null argument");
   if (n > e->cfg.max_batch_recs) return fail(GPX_ERANGE, "n > max_batch_recs");
-  int rc = ring_fits(e, 64ull + 32ull * n);
+  const LogSegs segs = one_seg(seg_decision_bytes(n));
+  int rc = ring_fits(e, segs);
   if (rc) return rc;
   cudaStream_t st = stream ? (cudaStream_t)stream : e->stream;
   {
@@ -1282,8 +1282,8 @@ int gpx_decisions_device(gpx_engine* e, gpx_decision_rec* decisions, uint32_t n,
     R.n = n;
     k_ingest<<<cdiv(n, GPX_BLOCK), GPX_BLOCK, 0, st>>>(e->S, R);
   }
-  ScratchSwap sw(e, ctl, nullptr, out_extra, out_extra ? extra_cap : 0);
-  return launch_commit(e, decisions, nullptr, n, out_exec, st);
+  log_advance(e, segs);
+  return launch_commit(e, e->sink(ctl, out_extra, extra_cap), decisions, nullptr, n, out_exec, st);
 }
 
 /* ---- pipelined rounds ---------------------------------------------------------------- */
@@ -1322,8 +1322,8 @@ int gpx_round_submit(gpx_engine* e, const gpx_round_io* io, uint64_t* ticket) {
   int rc = check_batch(e, n, io->payload_bytes);
   if (rc) return rc;
   const uint64_t pal = (io->payload_bytes + 15) & ~15ull;
-  const uint64_t b1 = e->cfg.batching_enabled ? std::min<uint64_t>(e->blob1_cap, 16ull * n + pal) : 0;
-  rc = ring_fits(e, 192ull + 80ull * n + pal + b1);
+  const LogSegs segs = round_segs(e, RoundForm::FUSED, n, io->payload_bytes);
+  rc = ring_fits(e, segs);
   if (rc) return rc;
   rc = pipe_init(e);
   if (rc) return rc;
@@ -1353,6 +1353,7 @@ int gpx_round_submit(gpx_engine* e, const gpx_round_io* io, uint64_t* ticket) {
     k_unpack_expand<<<nb, GPX_BLOCK, 0, e->stream>>>(e->S, ps.d_packed, n, ps.d_bsum, ps.d_reqs);
     CK(cudaGetLastError());
   }
+  log_advance(e, segs);
   rc = launch_round(e, ps.d_reqs, ps.d_payload, pal, n, ps.d_status, ps.d_exec, e->stream, ps.d_ctl, ps.d_extra,
                     (uint32_t)std::min<uint64_t>((uint64_t)e->cfg.max_batch_recs * (L + 1), 0xffffffffull),
                     compact ? ps.d_sum : nullptr);
@@ -1429,10 +1430,10 @@ int gpx_log_read(gpx_engine* e, uint32_t lane, uint64_t from, void* dst, uint64_
                  uint64_t* head) {
   if (!e) return fail(GPX_EINVAL, "null argument");
   if (lane >= e->cfg.n_lanes) return fail(GPX_ERANGE, "lane");
-  CK(cudaDeviceSynchronize());
-  unsigned long long pos[2 * GPX_MAX_LANES];
-  CK(cudaMemcpy(pos, e->S.log_pos + (size_t)e->S.lp * 2 * GPX_MAX_LANES, sizeof pos, cudaMemcpyDeviceToHost));
-  const uint64_t h = pos[2 * lane], rc = e->S.ring_cap;
+  uint64_t heads[GPX_MAX_LANES];
+  int err = read_device_heads(e, heads);
+  if (err) return err;
+  const uint64_t h = heads[lane], rc = e->S.ring_cap;
   if (head) *head = h;
   uint64_t nb = 0;
   if (dst && from < h) {
@@ -1505,10 +1506,10 @@ int gpx_log_gather(gpx_engine* e, uint32_t lane, uint32_t n, const gpx_log_range
   if (lane >= e->cfg.n_lanes) return fail(GPX_ERANGE, "lane");
   if (n == 0) return GPX_OK;
   if (!ranges || !dst) return fail(GPX_EINVAL, "null argument");
-  CK(cudaDeviceSynchronize());
-  unsigned long long lp[2 * GPX_MAX_LANES];
-  CK(cudaMemcpy(lp, e->S.log_pos + (size_t)e->S.lp * 2 * GPX_MAX_LANES, sizeof lp, cudaMemcpyDeviceToHost));
-  const uint64_t head = lp[2 * lane], cap = e->S.ring_cap;
+  uint64_t heads[GPX_MAX_LANES];
+  int rc = read_device_heads(e, heads);
+  if (rc) return rc;
+  const uint64_t head = heads[lane], cap = e->S.ring_cap;
   std::vector<uint32_t> first(n + 1);
   uint64_t chunks = 0, top = 0;
   for (uint32_t i = 0; i < n; i++) {
@@ -1526,7 +1527,7 @@ int gpx_log_gather(gpx_engine* e, uint32_t lane, uint32_t n, const gpx_log_range
   if (chunks == 0) return GPX_OK;
   const size_t r_bytes = ((size_t)n * sizeof(gpx_log_range) + 15) & ~(size_t)15;
   const size_t f_bytes = ((size_t)(n + 1) * 4 + 15) & ~(size_t)15;
-  int rc = e->ensure_misc(r_bytes + f_bytes + top);
+  rc = e->ensure_misc(r_bytes + f_bytes + top);
   if (rc) return rc;
   cudaStream_t st = e->stream;
   uint8_t* base = (uint8_t*)e->d_misc;

@@ -893,8 +893,8 @@ __global__ void __launch_bounds__(GPX_BLOCK, GPX_PHASE_MINB) k_accept(const __gr
   if (threadIdx.x == 0 && tile_bytes) tma_load_1d(s_tile, &A.recs[t0], tile_bytes, &s_bar);
   const uint32_t Wm = S.W - 1;
   const unsigned long long pay_bytes = A.blob0_bytes + (A.blob1_used_ptr ? *A.blob1_used_ptr : A.blob1_bytes);
-  const unsigned long long pay_rel = 64ull + (unsigned long long)A.n_max * 48ull;
-  const unsigned long long reserved = (pay_rel + pay_bytes + 31ull) & ~31ull; /* images need 32-B alignment */
+  const unsigned long long pay_rel = seg_pay_rel(A.n_max);
+  const unsigned long long reserved = seg_align32(pay_rel + pay_bytes); /* = seg_accept_bytes(A.n_max, pay_bytes) */
   unsigned long long segb[L], payb[L];
 #pragma unroll
   for (int l = 0; l < L; l++) {
@@ -1229,7 +1229,7 @@ __global__ void __launch_bounds__(GPX_BLOCK, 2) k_commit(const __grid_constant__
   if (n > A.n_max) n = A.n_max;
   const uint32_t i = blockIdx.x * GPX_BLOCK + threadIdx.x;
   const uint32_t Wm = S.W - 1;
-  const unsigned long long reserved = 64ull + (unsigned long long)A.n_max * 32ull;
+  const unsigned long long reserved = seg_decision_bytes(A.n_max);
   unsigned long long segb[L];
 #pragma unroll
   for (int l = 0; l < L; l++) segb[l] = seg_base(S, l, reserved);
@@ -1318,9 +1318,10 @@ __global__ void __launch_bounds__(GPX_BLOCK, GPX_ACT_MINB) k_act(const __grid_co
   const uint32_t i = blockIdx.x * GPX_BLOCK + threadIdx.x;
   const uint32_t Wm = S.W - 1;
   const unsigned long long pay_bytes = A.blob0_bytes + (A.blob1_used_ptr ? *A.blob1_used_ptr : A.blob1_bytes);
+  /* = seg_pay_rel(A.n_max), written out: calling the helper here reorders k_act's prologue */
   const unsigned long long pay_rel = 64ull + (unsigned long long)A.n_max * 48ull;
-  const unsigned long long res_a = (pay_rel + pay_bytes + 31ull) & ~31ull;
-  const unsigned long long res_d = 64ull + (unsigned long long)A.n_max * 32ull;
+  const unsigned long long res_a = seg_align32(pay_rel + pay_bytes); /* = seg_accept_bytes(A.n_max, pay_bytes) */
+  const unsigned long long res_d = seg_decision_bytes(A.n_max);
   unsigned long long segb[L], payb[L], dsegb[L];
 #pragma unroll
   for (int l = 0; l < L; l++) {

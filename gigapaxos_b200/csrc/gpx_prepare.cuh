@@ -23,7 +23,7 @@ __global__ void __launch_bounds__(GPX_BLOCK) k_prepare(const __grid_constant__ D
                                                        const __grid_constant__ PrepareArgs A) {
   const uint32_t n = A.n;
   const uint32_t i = blockIdx.x * GPX_BLOCK + threadIdx.x;
-  const unsigned long long reserved = 64ull + (unsigned long long)n * 32ull;
+  const unsigned long long reserved = seg_decision_bytes(n);
   unsigned long long segb[L];
 #pragma unroll
   for (int l = 0; l < L; l++) segb[l] = seg_base(S, l, reserved);

@@ -51,9 +51,9 @@ struct RoundArgs {
                                  * 0: the host launches k_round_slow behind every k_round */
   /* launch constants of the two log segments of a lane (host-computed: no 64-bit arithmetic in the kernels) */
   unsigned long long pay_bytes; /* payload area of the ACCEPT segment = blob0_bytes + blob1_res */
-  unsigned long long res_a;     /* ACCEPT segment bytes  = align32(64 + 48 n + pay_bytes) */
-  unsigned long long res_d;     /* DECISION segment bytes = 64 + 32 n */
-  uint32_t pay_rel;             /* payload area offset inside the ACCEPT segment = 64 + 48 n */
+  unsigned long long res_a;     /* ACCEPT segment bytes  = seg_accept_bytes(n, pay_bytes) (gpx_logseg.cuh) */
+  unsigned long long res_d;     /* DECISION segment bytes = seg_decision_bytes(n) */
+  uint32_t pay_rel;             /* payload area offset inside the ACCEPT segment = seg_pay_rel(n) */
   gpx_exec_sum* sum;            /* compact output mode (GPX_ROUND_COMPACT): one summary per request index instead of
                                  * n_lanes EXEC rows; everything that is not the plain in-order case goes to the
                                  * extra queue.  null = full EXEC rows */

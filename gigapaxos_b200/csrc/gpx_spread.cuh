@@ -240,8 +240,8 @@ __global__ void __launch_bounds__(GPX_BLOCK, GPX_PHASE_MINB) k_sp_accept(const _
   if (threadIdx.x == 0 && tile_bytes) tma_load_1d(s_tile, &recs[t0], tile_bytes, &s_bar);
   const uint32_t Wm = S.W - 1;
   /* one ACCEPT segment per round: an image slot per virtual index, payload area = the received blob areas */
-  const unsigned long long pay_rel = 64ull + (unsigned long long)A.vtotal * 48ull;
-  const unsigned long long reserved = (pay_rel + A.blob_vtotal + 31ull) & ~31ull;
+  const unsigned long long pay_rel = seg_pay_rel(A.vtotal);
+  const unsigned long long reserved = seg_align32(pay_rel + A.blob_vtotal); /* = seg_accept_bytes(A.vtotal, blob_vtotal) */
   const unsigned long long segb = seg_base(S, 0, reserved);
   const unsigned long long payb = segb + pay_rel + B.blob_off;
   if (v == 0) {
@@ -447,7 +447,7 @@ __global__ void __launch_bounds__(GPX_BLOCK, GPX_PHASE_MINB) k_sp_commit(const _
   if (cnt > B.cap) cnt = B.cap;
   const gpx_decision_rec* recs = reinterpret_cast<const gpx_decision_rec*>(sp_recs(B));
   const uint32_t Wm = S.W - 1;
-  const unsigned long long reserved = 64ull + (unsigned long long)A.vtotal * 32ull;
+  const unsigned long long reserved = seg_decision_bytes(A.vtotal);
   const unsigned long long segb = seg_base(S, 0, reserved);
   if (v == 0) {
     const unsigned long long sq = seg_seq_of(S, 0);
